@@ -7,7 +7,7 @@ on one synthetic 64k-point Velodyne sweep against a 1M-point map (BASELINE.json 
 config/xaloc.yaml).  Prints ONE JSON line (see the task contract); `--impl reference` times the CPU
 oracle (reference ikd-Tree compiled verbatim into oracle/_ref + restated plane/Jacobian/IESKF).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR]
 """
 import argparse
 import json
@@ -353,6 +353,8 @@ def run_native(args, rank, local_rank, world_size):
     launches = loc.profile(reset=True)["total_launches"]
     step_ms = sum(a.elapsed_time(b) for a, b in evs)
     pts = n * evals
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loc)
 
     # ---- per-kernel device time (roofline): the same steps again with CUDA events around each kernel group.
     # The timed region above replays an update as ONE CUDA graph; events between its kernels would add bubbles,
@@ -573,6 +575,20 @@ def run_native(args, rank, local_rank, world_size):
         dist.destroy_process_group()
 
 
+def dump_outputs(out_dir, loc):
+    """What the last timed step handed its caller (lv_last_logs, lv_get_state), as DIR/<name>.npy in float64: the
+    status, the per-evaluation logs stacked along axis 0, and the updated state x (26) and covariance P (23 x 23).
+    The inputs are seeded, so two builds run with the same arguments can be compared file by file."""
+    st, logs = loc.last_logs()
+    x, P = loc.get_state()
+    out = {"status": [st], "x": x, "P": P}
+    for k in ("n_matches", "converged", "degenerate", "HTH", "HTh", "dx", "x_after"):
+        out[k] = [lg[k] for lg in logs]
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), np.asarray(v, dtype=np.float64))
+
+
 def multi_sequence_leg(lv, torch, cfg, local_rank, rank, s_list, steps):
     """point-evaluations/s of ONE GPU running S independent sequences at once (S handles, S streams, no shared state)"""
     out = []
@@ -780,7 +796,14 @@ def main():
     ap.add_argument("--sequences-per-gpu", default="", help="e.g. 1,2,4,8: also measure S concurrent sequences per GPU (multi_sequence)")
     ap.add_argument("--sort-queries", type=int, default=None, help="tuning: 1 = binned order + search from shared memory, 0 = per-query search")
     ap.add_argument("--voxel", type=float, default=0.0, help="tuning: finest voxel edge of the map (0 = library default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the last step's results (state, covariance, per-evaluation logs) "
+                         "as DIR/<name>.npy (float64, about 20 KB; rank 0's sequence)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "native" or args.config == "cfg4"):
+        ap.error("--dump-outputs writes the native single-sequence update (--impl native, --config cfg0..cfg3)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world_size = int(os.environ.get("WORLD_SIZE", "1"))

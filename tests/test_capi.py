@@ -8,6 +8,7 @@ import re
 import numpy as np
 import pytest
 
+import reference_golden as RG
 from conftest import have_gpu
 
 
@@ -100,11 +101,11 @@ def test_yaml_reader_matches_pyyaml(lv):
         assert p.covariance_bias_acceleration == float(ref["covariance_bias_acceleration"])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/config"), reason="reference tree not mounted")
 def test_yaml_reader_on_the_reference_configs(lv):
-    """the full ROS config files of the reference parse to the same hot-path values as our subsets"""
+    """the full ROS config files of the reference (tests/golden/reference/config) parse to the same hot-path values as
+    our subsets"""
     for name in ("xaloc.yaml", "kitti.yaml", "ouster.yaml"):
-        a = lv.params_from_yaml(os.path.join("/root/reference/config", name))
+        a = lv.params_from_yaml(os.path.join(RG.CONFIG_DIR, name))
         b = lv.params_from_yaml(os.path.join(lv.CONFIG_DIR, name))
         for f in ("MAX_NUM_ITERS", "NUM_MATCH_POINTS", "estimate_extrinsics", "MAX_DIST_PLANE", "PLANES_THRESHOLD",
                   "LiDAR_noise", "degeneracy_threshold", "covariance_gyroscope", "covariance_acceleration",

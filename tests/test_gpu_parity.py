@@ -7,6 +7,7 @@ accept decision) must be BIT-EXACT; the fp64 rows of H are bit-exact; reduced su
 import numpy as np
 import pytest
 
+import reference_golden as RG
 from conftest import Scene
 
 pytestmark = pytest.mark.gpu
@@ -39,14 +40,16 @@ def test_match_all_bit_exact(lv, O, name, request):
 
 
 def test_match_against_reference_ikdtree(lv, O, scene_xaloc):
-    """neighbour distances/coordinates equal those of the reference's own ikd-Tree (oracle/_ref)"""
-    if not O.ref_available():
-        pytest.skip("oracle/_ref not built")
+    """neighbour distances/coordinates equal those of the reference's own ikd-Tree (stored as digests, see
+    tests/reference_golden.py: the oracle reproduces them bit for bit and stands in for the reference below)"""
     sc = scene_xaloc
+    golden = RG.load()
+    RG.check_scene(golden, sc)
+    ref = _oracle_map(O, sc).match_all(sc.x_prop, sc.oprm, sc.sweep)
+    assert [RG.digest(ref[k]) for k in RG.MATCH_FIELDS] == golden["xaloc_match"].tolist()
     loc = lv.Localizer(sc.prm)
     loc.map_build(sc.map)
     got = loc.match_all(sc.x_prop, sc.sweep)
-    ref = _oracle_map(O, sc, O.KNN_REF_IKDTREE).match_all(sc.x_prop, sc.oprm, sc.sweep)
     inside = np.isfinite(got["nn_sqd"][:, 4])
     assert (got["nn_sqd"][inside] == ref["nn_sqd"][inside]).all()
     assert (got["valid"] == ref["valid"]).all()
@@ -181,17 +184,18 @@ def test_map_build_roundtrip_and_add(lv, O, scene_xaloc):
     R = O.quat_to_rot(sc.truth[3:7]); RL = O.quat_to_rot(sc.truth[7:11])
     new = ((sc.sweep.astype(np.float64) @ RL.T + sc.truth[11:14]) @ R.T + sc.truth[0:3]).astype(np.float32)
     loc.map_add(new, downsample=True)
-    backends = [O.KNN_KDTREE] + ([O.KNN_REF_IKDTREE] if O.ref_available() else [])
     got = loc.map_points()
     got_set = set(map(tuple, got.tolist()))
     assert len(got_set) == len(got)
-    for be in backends:
-        om = O.Map(be)
-        om.build(sc.map)
-        om.add(new, downsample=True)
-        ref_set = set(map(tuple, om.points().tolist()))
-        diff = len(got_set ^ ref_set)
-        assert diff <= 1e-4 * len(ref_set), (be, diff, len(got_set), len(ref_set))
+    om = O.Map(O.KNN_KDTREE)
+    om.build(sc.map)
+    om.add(new, downsample=True)
+    golden = RG.load()
+    RG.check_scene(golden, sc)
+    assert RG.set_digest(om.points()) == golden["xaloc_add"]         # the oracle holds what the reference ikd-Tree holds
+    ref_set = set(map(tuple, om.points().tolist()))
+    diff = len(got_set ^ ref_set)
+    assert diff <= 1e-4 * len(ref_set), (diff, len(got_set), len(ref_set))
     # the rebuilt structure serves queries: parity after the add
     om = O.Map(O.KNN_KDTREE)
     om.build(got)

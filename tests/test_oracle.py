@@ -1,7 +1,7 @@
 """The CPU oracle pinned against what can be pinned here (SURVEY.md 8c):
 
-* its exact kNN and its Add_Points restatement against the reference's OWN ikd-Tree, compiled
-  verbatim from /root/reference into oracle/_ref (skipped where that build is absent);
+* its exact kNN and its Add_Points restatement against the reference's OWN ikd-Tree (its answers are stored
+  under tests/golden/reference, see tests/reference_golden.py);
 * its small dense algebra (LU inverse, symmetric 6x6 eigen, 5x3 least squares) against numpy/LAPACK;
 * its IESKF step against an independent numpy statement of esekfom.hpp:1722-1733;
 * manifold identities of the MTK restatement.
@@ -10,6 +10,8 @@ reproducible without Eigen ("parity unpinned" for that part, see oracle/lv_oracl
 """
 import numpy as np
 import pytest
+
+import reference_golden as RG
 
 
 def _cloud(seed, m, span=20.0):
@@ -20,17 +22,28 @@ def _cloud(seed, m, span=20.0):
     return np.vstack([a, b]).astype(np.float32)
 
 
-def test_knn_backends_agree(O):
+def _knn_case():
     pts = _cloud(1, 20000)
     rng = np.random.default_rng(2)
     q = (pts[rng.integers(0, len(pts), 300)] + rng.normal(0, 0.1, (300, 3))).astype(np.float32)
+    return pts, q
+
+
+def _add_case():
+    base = _cloud(3, 8000, span=6.0)
+    rng = np.random.default_rng(4)
+    new = (base[rng.integers(0, len(base), 3000)] + rng.normal(0, 0.05, (3000, 3))).astype(np.float32)
+    new2 = (new[:1500] + np.float32([0.03, -0.02, 0.01])).astype(np.float32)
+    return base, new, new2
+
+
+def test_knn_backends_agree(O):
+    pts, q = _knn_case()
+    golden = RG.load()
     maps = {}
     for name, be in (("brute", O.KNN_BRUTE), ("kd", O.KNN_KDTREE)):
         maps[name] = O.Map(be)
         maps[name].build(pts)
-    if O.ref_available():
-        maps["ref"] = O.Map(O.KNN_REF_IKDTREE)
-        maps["ref"].build(pts)
     for i in range(len(q)):
         fb, ib, db, nb = maps["brute"].knn(q[i])
         fk, ik, dk, nk = maps["kd"].knn(q[i])
@@ -41,9 +54,8 @@ def test_knn_backends_agree(O):
         d = q[i] - pts[ib]
         ref = (d[:, 0] * d[:, 0] + d[:, 1] * d[:, 1]) + d[:, 2] * d[:, 2]
         assert (ref.astype(np.float32) == db).all()
-        if "ref" in maps:
-            fr, _, dr, nr = maps["ref"].knn(q[i])
-            assert fr == 5 and (dr == db).all() and (nr == nb).all()
+        # the reference ikd-Tree's answer
+        assert golden["knn_found"][i] == 5 and (golden["knn_sqd"][i] == db).all() and (golden["knn_xyz"][i] == nb).all()
 
 
 def test_knn_fewer_points_than_k(O):
@@ -55,30 +67,22 @@ def test_knn_fewer_points_than_k(O):
 
 def test_map_add_matches_reference_ikdtree(O):
     """Add_Points with the 0.2 m voxel rule (ikd_Tree.cpp:478-573): oracle restatement vs the real thing."""
-    if not O.ref_available():
-        pytest.skip("oracle/_ref not built")
-    base = _cloud(3, 8000, span=6.0)
-    rng = np.random.default_rng(4)
-    new = (base[rng.integers(0, len(base), 3000)] + rng.normal(0, 0.05, (3000, 3))).astype(np.float32)
-    a, b = O.Map(O.KNN_KDTREE), O.Map(O.KNN_REF_IKDTREE)
-    for m in (a, b):
-        m.build(base)
-        m.add(new, downsample=True)
+    golden = RG.load()
+    base, new, new2 = _add_case()
+    a = O.Map(O.KNN_KDTREE)
+    a.build(base)
+    a.add(new, downsample=True)
     sa = set(map(tuple, a.points().tolist()))
-    sb = set(map(tuple, b.points().tolist()))
     # KD_TREE::size() counts lazily deleted nodes too (ikd_Tree.cpp size() = Root_Node->TreeSize), so
     # the CONTENT is compared through flatten (ikd_Tree.cpp:1626-1657), not through size()
-    assert a.size() == len(sa) == len(sb) and b.size() >= len(sb)
-    assert sa == sb
+    assert a.size() == len(sa) == golden["add_count"][0] and golden["add_tree_size"] >= len(sa)
+    assert RG.set_digest(a.points()) == golden["add_digest"][0]
     # a second batch on top (touched voxels collapse to one point)
-    new2 = (new[:1500] + np.float32([0.03, -0.02, 0.01])).astype(np.float32)
     a.add(new2, downsample=True)
-    b.add(new2, downsample=True)
-    assert set(map(tuple, a.points().tolist())) == set(map(tuple, b.points().tolist()))
+    assert RG.set_digest(a.points()) == golden["add_digest"][1]
     # without downsampling everything is kept
     a.add(new2, downsample=False)
-    b.add(new2, downsample=False)
-    assert len(a.points()) == len(b.points())
+    assert len(a.points()) == golden["add_count"][1]
 
 
 def test_dense_algebra_against_lapack(O):
