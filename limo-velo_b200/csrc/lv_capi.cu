@@ -213,7 +213,9 @@ extern "C" {
 
 const char* lv_last_error(void) { return g_last_error.c_str(); }
 const char* lv_version(void) { return "limovelo_b200 0.1 (sm_100a)"; }
-int64_t lv_result_bytes(void) { return (int64_t)sizeof(UpdateCtrl); }
+/* the results are UpdateCtrl up to `prep`, which only the kernels of an update read */
+static const size_t kResultBytes = offsetof(UpdateCtrl, prep);
+int64_t lv_result_bytes(void) { return (int64_t)kResultBytes; }
 
 /* every failure after `new lv_context` goes through here: nothing of a half-built context survives */
 #define LV_CREATE_CUDA(call)                                                                     \
@@ -662,7 +664,7 @@ static lv_status enqueue_update_kernels(lv_context* h, const float* d_xyz, int64
 }
 
 static lv_status fetch_results(lv_context* h) {
-    LV_CUDA(cudaMemcpyAsync(h->h_ctrl, h->d_ctrl, sizeof(UpdateCtrl), cudaMemcpyDeviceToHost, h->stream));
+    LV_CUDA(cudaMemcpyAsync(h->h_ctrl, h->d_ctrl, kResultBytes, cudaMemcpyDeviceToHost, h->stream));
     LV_CUDA(map_fetch_counters(h->map, h->stream));       /* 64 bytes: the map's error flags ride along */
     LV_CUDA(cudaStreamSynchronize(h->stream));
     const UpdateCtrl* c = h->h_ctrl;

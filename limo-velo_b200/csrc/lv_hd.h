@@ -20,9 +20,13 @@
 #if defined(__CUDACC__)
 #define LV_HD __host__ __device__ __forceinline__
 #define LV_HD_NOINLINE __host__ __device__ inline
+/* out of line on the device as well: rare or single-thread code that would otherwise take registers and
+ * instruction-cache space from the kernel it is called in */
+#define LV_HD_COLD __host__ __device__ inline __noinline__
 #else
 #define LV_HD inline
 #define LV_HD_NOINLINE inline
+#define LV_HD_COLD inline
 #endif
 
 namespace lv {

@@ -13,7 +13,7 @@
 
 namespace lv {
 
-enum { kMeasureThreads = 128, kPartialStride = 96, kStepThreads = 512, kPartialGroup = 32 };
+enum { kMeasureThreads = 128, kPartialStride = 96, kStepThreads = 256, kPartialGroup = 32 };
 inline int partial_groups(int grid) { return (grid + kPartialGroup - 1) / kPartialGroup; }
 /* The search kernel appends its uncertified queries to one of 32 lists picked by block index: thousands of atomics on
  * ONE counter cost it a 9 us tail on the first evaluation of an update (tools/timeline.py). */

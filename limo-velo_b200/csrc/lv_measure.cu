@@ -807,10 +807,14 @@ __device__ void reduce_partials_block(const double* partials, int n_partials, do
     __syncthreads();
 }
 
-__global__ void __launch_bounds__(kStepThreads) lv_ieskf_step_kernel(UpdateCtrl* c, const IeskfParams prm,
+__global__ void __launch_bounds__(kStepThreads, 1) lv_ieskf_step_kernel(UpdateCtrl* c, const IeskfParams prm,
                                                                      const double* partials, int n_partials) {
+    /* (min. blocks 1: the kernel runs as a single block, so ptxas may use up to 255 registers; with the default bound it
+     * stopped at 128 and spilled) */
     /* before the wait: what the previous step (or begin) kernel left, two or more kernels ago */
-    static_assert(kStepThreads >= 99 && 2 * kStepThreads >= kN * kN, "one pass for the state, two for P_j");
+    constexpr int kPrepWords = (int)(sizeof(StepPrep) / sizeof(double));
+    constexpr int kPrepLoads = (kPrepWords + kStepThreads - 1) / kStepThreads;
+    static_assert(kStepThreads >= 99, "one pass for the state and the counters");
     LV_TL_SCHED();
     const int t = threadIdx.x;
     const int done = c->done;
@@ -819,7 +823,7 @@ __global__ void __launch_bounds__(kStepThreads) lv_ieskf_step_kernel(UpdateCtrl*
     else if (t < 52) sv = c->x_prop[t - 26];
     int cv = 0;
     if (t >= 96 && t < 99) cv = t == 96 ? c->n_evals : (t == 97 ? c->t : c->iter);
-    pdl_wait();                 /* partials and the prepared P_j / dx_new of the fit kernel */
+    pdl_wait();                 /* partials and c->prep, written by the fit kernel */
     pdl_trigger();
     LV_TL_WORK(c, 5);
     if (done) return;
@@ -829,16 +833,18 @@ __global__ void __launch_bounds__(kStepThreads) lv_ieskf_step_kernel(UpdateCtrl*
     LV_CK(0);
     /* ieskf_load(), split: the loads are issued here and parked in shared memory after the reduction, so
      * they are in flight together with the partials */
-    const double pj0 = t < kN * kN ? c->P_j[t] : 0.0;
-    const double pj1 = t + kStepThreads < kN * kN ? c->P_j[t + kStepThreads] : 0.0;
-    if (t >= 52 && t < 75) sv = c->dx_new[t - 52];
+    const double* src = reinterpret_cast<const double*>(&c->prep);
+    double pv[kPrepLoads];
+#pragma unroll
+    for (int r = 0; r < kPrepLoads; ++r) pv[r] = t + r * kStepThreads < kPrepWords ? src[t + r * kStepThreads] : 0.0;
     LV_CK(1);
     reduce_partials_block(partials, n_partials, s_tmp, w.HTH, w.HTh, &w.n_matches);
-    if (t < kN * kN) w.P[t] = pj0;
-    if (t + kStepThreads < kN * kN) w.P[t + kStepThreads] = pj1;
+    double* dst = reinterpret_cast<double*>(&w.p);
+#pragma unroll
+    for (int r = 0; r < kPrepLoads; ++r)
+        if (t + r * kStepThreads < kPrepWords) dst[t + r * kStepThreads] = pv[r];
     if (t < 26) w.x[t] = sv;
     else if (t < 52) w.xp[t - 26] = sv;
-    else if (t < 75) w.dx_new[t - 52] = sv;
     if (t == 96) { w.n_evals = cv; w.eval_idx = cv < kMaxEvals ? cv : kMaxEvals - 1; }
     if (t == 97) w.t = cv;
     if (t == 98) w.iter = cv;

@@ -22,5 +22,5 @@ for it in range(12):
     print(("flush " if it % 2 else "warm  ") + " ".join(f"{d:7d}" for d in ph), " total", b[9] - b[0], " non-final", b[8] - b[0],
           " T1 tasks (pose, extr, grav, lin+conv):", [b[32 + k] - b[24 + k] for k in range(4)],
           " FIT block 1 (cycles): wait", b[57] - b[56], "loads", b[58] - b[57], "fit+row", b[59] - b[58], "stage", b[60] - b[59], "reduce", b[61] - b[60], "store+ticket", b[62] - b[61], "group sum", b[63] - b[62], "|",
-          " gj: entry->loop", b[48] - b[5], "loop", b[49] - b[48], "store", b[52] - b[49], "exit->CK6", b[6] - b[52], " chol", b[51] - b[50])
-print("phases: load | reduce | M1 | gj(+chol) | K,dxs | tail | exit-P")
+          " solve: entry->loop", b[48] - b[5], "loop", b[49] - b[48], "store", b[52] - b[49], "exit->CK6", b[6] - b[52], " degeneracy test", b[51] - b[50])
+print("phases: load | reduce | assemble A | solve (+degeneracy test) | K,dxs | tail | exit-P")
